@@ -8,6 +8,7 @@ per GPU, DDPM with 1000 steps per mel-spectrogram.  value = (batch * n_gpus) / (
     python bench.py --gpus N --steps K --warmup W            # B200 arm (libb200ad.so)
     python bench.py --impl reference --gpus N ...            # CPU arm: oracle port of diffusers, host cores
     python bench.py --mode train ...                         # only the train_unet.py iteration (config C5)
+    python bench.py ... --dump-outputs DIR                   # also save the sample the last timed step returned (.npy)
 
 The JSON line of the default arm also carries
   e2e         whole `AudioDiffusionPipeline.__call__` (host noise in, PIL images + audio out): ONE complete 1000-step call
@@ -31,6 +32,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True             # the tree may be read-only: no __pycache__ for the modules imported from it
 if os.environ.get("NCCL_DEBUG", "").upper() == "VERSION":
     os.environ["NCCL_DEBUG"] = "WARN"      # before torch loads NCCL: its version banner goes to STDOUT, next to the one JSON line
 
@@ -257,6 +259,9 @@ def run_b200(args):
         ms = e0.elapsed_time(e1) / K
         clocks = sampler.stop()
         launches = model.last_launch_count * K
+        if args.dump_outputs and rank == 0:
+            # the sample the last timed step returned, before the passes below reuse its buffer
+            dump_outputs(args.dump_outputs, {"sample": x})
 
         # ---- e2e: AudioDiffusionPipeline.__call__ — pinned host noise in (H2D inside), K denoise steps incl. the per-step
         # noise draw, float->uint8, D2H, PIL, batched Griffin-Lim, audio D2H.  Two step counts separate the per-step cost
@@ -391,6 +396,23 @@ def run_b200(args):
     print(json.dumps(line), flush=True)
     if use_dist:
         dist.destroy_process_group()
+
+
+MAX_DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(d, arrays):
+    """Write each tensor as d/<name>.npy in float32.  A tensor over MAX_DUMP_BYTES keeps a fixed, seeded choice of whole
+    samples along dim 0 (the same rows on every run), so that two builds can be compared output for output."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    for name, t in arrays.items():
+        per = t[0].numel() * 4
+        if t.shape[0] * per > MAX_DUMP_BYTES:
+            keep = max(MAX_DUMP_BYTES // per, 1)
+            rows = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            t = t[rows.to(t.device)]
+        np.save(os.path.join(d, name + ".npy"), t.float().cpu().numpy())
 
 
 def parity_check(model, sch, B, HW, dev):
@@ -703,7 +725,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline and parity_check legs (both run the CPU oracle)")
     ap.add_argument("--no-extras", action="store_true", help="skip the C3/C4/C5/Mel sub-benchmarks and the sustained call")
     ap.add_argument("--dump-ops", default=None, help="write the per-launch profile (kind, ms, flops) to this JSON")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps write the sample the last one returned (rank 0) as DIR/sample.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.mode != "sample"):
+        ap.error("--dump-outputs writes the outputs of the B200 sampling path (--impl b200 --mode sample)")
     if os.environ.get("NCCL_DEBUG", "").upper() == "VERSION":
         os.environ["NCCL_DEBUG"] = "WARN"      # keep stdout to the one JSON line (NCCL prints its version banner to stdout)
     if args.impl == "reference":

@@ -1,9 +1,12 @@
-"""CPU tests of the drop-in boundary: the UNCHANGED reference pipeline file runs on top of the import shim
-(`audio_diffusion_b200/compat`) with the product's schedulers / pipeline base, and the N>1 path's host logic
-(weight broadcast + batch sharding) works over gloo with world_size 2.
+"""CPU tests of the drop-in boundary: the product's pipeline, schedulers, Mel, VAE loader and import shim
+(`audio_diffusion_b200/compat`) against what the UNCHANGED reference files compute, and the N>1 path's host logic
+(weight broadcast + batch sharding) over gloo with world_size 2.
 
-The reference sources are read from /root/reference when present (this container); on the GPU box the test skips.
+The reference's results are stored under tests/golden/ (written by tests/golden/make_golden.py, which runs the reference
+files on the import shim); these tests need no reference checkout.
 """
+import hashlib
+import json
 import os
 import subprocess
 import sys
@@ -13,7 +16,7 @@ import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 
 class OracleUNet:
@@ -43,40 +46,50 @@ class FakeMel:
         return np.zeros((self.x_res - 1) * self.hop_length, dtype=np.float32)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference sources not present (GPU box)")
+def _golden_images(key):
+    return np.load(os.path.join(GOLDEN, "reference_pipeline_cpu.npz"))[key]
+
+
+def _host_u8_pipeline(monkeypatch):
+    """The product's AudioDiffusionPipeline with its float->uint8 CUDA kernel replaced by the same torch expression, so
+    that it runs on the CPU around the oracle U-Net (it then takes its unfused branch)."""
+    from audio_diffusion_b200.pipeline import AudioDiffusionPipeline
+    monkeypatch.setattr(AudioDiffusionPipeline, "images_to_u8",
+                        staticmethod(lambda x: ((x / 2 + 0.5).clamp(0, 1) * 255).round().to(torch.uint8)))
+    return AudioDiffusionPipeline
+
+
+def _scheduler(sched):
+    from audio_diffusion_b200.schedulers import DDIMScheduler, DDPMScheduler
+    return DDIMScheduler() if sched == "ddim" else DDPMScheduler()
+
+
 @pytest.mark.parametrize("sched", ["ddpm", "ddim"])
-def test_unchanged_reference_pipeline_runs_on_the_shim(sched):
-    code = f"""
-import sys
-sys.path[:0] = [{ROOT!r}, {os.path.join(ROOT, 'audio_diffusion_b200', 'compat')!r}, {REF!r}, {os.path.join(ROOT, 'tests')!r}]
-import torch, numpy as np
-from audiodiffusion.pipeline_audio_diffusion import AudioDiffusionPipeline as RefPipe   # byte-identical reference file
-from diffusers import DDPMScheduler, DDIMScheduler
-from test_cpu_dropin import OracleUNet, FakeMel
-from oracle.schedulers_oracle import OracleDDPM, OracleDDIM
-from oracle.unet_oracle import unet_forward
-is_ddim = {sched!r} == 'ddim'
-unet = OracleUNet()
-pipe = RefPipe(vqvae=None, unet=unet, mel=FakeMel(), scheduler=(DDIMScheduler() if is_ddim else DDPMScheduler()))
-assert pipe.get_default_steps() == (50 if is_ddim else 1000)
-pipe.set_progress_bar_config(disable=True)
-out = pipe(batch_size=2, steps=4, generator=torch.Generator().manual_seed(42))
-assert len(out.images) == 2 and out.images[0].size == (16, 16) and out.audios.shape == (2, 1, 15 * 512)
-# same loop by hand with the oracle schedulers -> identical uint8 images
-g = torch.Generator().manual_seed(42)
-x = torch.randn((2, 1, 16, 16), generator=g)
-o = OracleDDIM() if is_ddim else OracleDDPM()
-o.set_timesteps(4)
-for t in o.timesteps:
-    eps = unet_forward(unet.w, unet.cfg, x, t)
-    x = (o.step(eps, t, x, eta=0, generator=g) if is_ddim else o.step(eps, t, x, generator=g))['prev_sample']
-ref = ((x / 2 + 0.5).clamp(0, 1).permute(0, 2, 3, 1).numpy() * 255).round().astype('uint8')[..., 0]
-got = np.stack([np.asarray(im) for im in out.images])
-assert np.array_equal(got, ref), np.abs(got.astype(int) - ref.astype(int)).max()
-print('ok')
-"""
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
-    assert r.returncode == 0 and "ok" in r.stdout, r.stderr[-2000:]
+def test_unchanged_reference_pipeline_runs_on_the_shim(sched, monkeypatch):
+    """`shim_<sched>` of tests/golden/reference_pipeline_cpu.npz holds the images the unchanged reference pipeline file
+    returned on the import shim (the product's schedulers, the CPU oracle U-Net, batch 2, 4 steps, generator seed 42).
+    The same loop by hand with the oracle schedulers, and the product's own pipeline on the same call, give those bytes."""
+    from oracle.schedulers_oracle import OracleDDIM, OracleDDPM
+    from oracle.unet_oracle import unet_forward
+    gold = _golden_images(f"shim_{sched}")
+    is_ddim = sched == "ddim"
+    unet = OracleUNet()
+    g = torch.Generator().manual_seed(42)
+    x = torch.randn((2, 1, 16, 16), generator=g)
+    o = OracleDDIM() if is_ddim else OracleDDPM()
+    o.set_timesteps(4)
+    for t in o.timesteps:
+        eps = unet_forward(unet.w, unet.cfg, x, t)
+        x = (o.step(eps, t, x, eta=0, generator=g) if is_ddim else o.step(eps, t, x, generator=g))["prev_sample"]
+    ref = ((x / 2 + 0.5).clamp(0, 1).permute(0, 2, 3, 1).numpy() * 255).round().astype("uint8")[..., 0]
+    assert np.array_equal(gold, ref), np.abs(gold.astype(int) - ref.astype(int)).max()
+    pipe = _host_u8_pipeline(monkeypatch)(vqvae=None, unet=unet, mel=FakeMel(), scheduler=_scheduler(sched))
+    assert pipe.get_default_steps() == (50 if is_ddim else 1000)
+    pipe.set_progress_bar_config(disable=True)
+    out = pipe(batch_size=2, steps=4, generator=torch.Generator().manual_seed(42))
+    assert len(out.images) == 2 and out.images[0].size == (16, 16) and out.audios.shape == (2, 1, 15 * 512)
+    got = np.stack([np.asarray(im) for im in out.images])
+    assert np.array_equal(got, gold), np.abs(got.astype(int) - gold.astype(int)).max()
 
 
 def _worker(rank, world, port, q):
@@ -139,36 +152,29 @@ def _hf_to_ldm_vae(w, num_blocks=4):
     return out
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference sources not present (GPU box)")
 def test_reference_vae_converter_feeds_the_b200_autoencoder():
-    """audiodiffusion/utils.py:156-291 (`convert_ldm_vae_checkpoint`, UNCHANGED, imported through the shim) turns an
-    ldm-format checkpoint into exactly the state dict the B200 `AutoencoderKL` loads: the library's parameter table
-    (names and shapes) is pinned against the reference's own converter."""
-    code = f"""
-import sys
-sys.path[:0] = [{ROOT!r}, {os.path.join(ROOT, 'audio_diffusion_b200', 'compat')!r}, {REF!r}, {os.path.join(ROOT, 'tests')!r}]
-import torch
-from audiodiffusion.utils import convert_ldm_vae_checkpoint            # byte-identical reference file
-from diffusers import AutoencoderKL                                     # -> audio_diffusion_b200.vae.AutoencoderKL
-from oracle.vae_oracle import VAEConfig, init_weights
-from test_cpu_dropin import _hf_to_ldm_vae
-w = init_weights(VAEConfig(), seed=3)
-ldm = _hf_to_ldm_vae(w)
-assert any(k.startswith('encoder.down.0.block.0.') for k in ldm) and 'decoder.mid.attn_1.q.weight' in ldm
-assert ldm['decoder.mid.attn_1.q.weight'].dim() == 4
-conv = convert_ldm_vae_checkpoint(dict(ldm), None)
-vae = AutoencoderKL(in_channels=1, out_channels=1, down_block_types=('DownEncoderBlock2D',) * 4,
-                    up_block_types=('UpDecoderBlock2D',) * 4, block_out_channels=(128, 256, 512, 512),
-                    layers_per_block=2, latent_channels=1)
-vae.load_state_dict(conv)                                               # strict: every key must land
-sd = vae.state_dict()
-assert set(sd) == set(w)
-for k in w:
-    assert torch.equal(sd[k], w[k]), k
-print('OK', len(sd))
-"""
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0 and "OK 248" in r.stdout, r.stdout + r.stderr
+    """audiodiffusion/utils.py:156-291 (`convert_ldm_vae_checkpoint`, UNCHANGED) turns an ldm-format checkpoint into
+    exactly the state dict the B200 `AutoencoderKL` loads.  The converter's key mapping (ldm key -> hf key and shape, read
+    off the reference by tests/golden/make_golden.py into vae_ldm_to_hf.json) is applied to an ldm checkpoint and the
+    result must load strictly and give back every original tensor."""
+    from audio_diffusion_b200.vae import AutoencoderKL                     # what the shim's `diffusers.AutoencoderKL` is
+    from oracle.vae_oracle import VAEConfig, init_weights
+    w = init_weights(VAEConfig(), seed=3)
+    ldm = _hf_to_ldm_vae(w)
+    assert any(k.startswith("encoder.down.0.block.0.") for k in ldm) and "decoder.mid.attn_1.q.weight" in ldm
+    assert ldm["decoder.mid.attn_1.q.weight"].dim() == 4
+    with open(os.path.join(GOLDEN, "vae_ldm_to_hf.json")) as f:
+        mapping = json.load(f)["map"]
+    assert {old for old, _, _ in mapping} == set(ldm)
+    conv = {new: ldm[old].reshape(shape) for old, new, shape in mapping}
+    vae = AutoencoderKL(in_channels=1, out_channels=1, down_block_types=("DownEncoderBlock2D",) * 4,
+                        up_block_types=("UpDecoderBlock2D",) * 4, block_out_channels=(128, 256, 512, 512),
+                        layers_per_block=2, latent_channels=1)
+    vae.load_state_dict(conv)                                               # strict: every key must land
+    sd = vae.state_dict()
+    assert set(sd) == set(w) and len(sd) == 248
+    for k in w:
+        assert torch.equal(sd[k], w[k]), k
 
 
 def test_gradient_allreduce_gloo_world2():
@@ -253,103 +259,106 @@ class ScriptedMel(FakeMel):
         return Image.fromarray(rng.integers(0, 256, (self.y_res, self.x_res), dtype=np.uint8))
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference sources not present (GPU box)")
-@pytest.mark.parametrize("sched", ["ddpm", "ddim"])
-def test_mirrored_pipeline_equals_reference_pipeline_on_cpu(sched):
-    """The product's own `AudioDiffusionPipeline.__call__` (audio_diffusion_b200/pipeline.py) against the reference's
-    unchanged file for the audio-conditioned / in-painting path (`raw_audio`, `start_step`, `mask_start_secs`,
-    `mask_end_secs`, pipeline_audio_diffusion.py:133-185): identical uint8 images. Both drive the CPU oracle U-Net (the mirror
-    then takes its unfused branch); only the mirror's float->uint8 CUDA kernel is replaced by the same torch expression."""
-    code = f"""
-import sys
-sys.path[:0] = [{ROOT!r}, {os.path.join(ROOT, 'audio_diffusion_b200', 'compat')!r}, {REF!r}, {os.path.join(ROOT, 'tests')!r}]
-import torch, numpy as np
-from audiodiffusion.pipeline_audio_diffusion import AudioDiffusionPipeline as RefPipe   # byte-identical reference file
-from audio_diffusion_b200.pipeline import AudioDiffusionPipeline as Mirror
-from diffusers import DDPMScheduler, DDIMScheduler
-from test_cpu_dropin import OracleUNet, ScriptedMel
-Mirror.images_to_u8 = staticmethod(lambda x: ((x / 2 + 0.5).clamp(0, 1) * 255).round().to(torch.uint8))
-is_ddim = {sched!r} == 'ddim'
-outs = []
-for cls in (RefPipe, Mirror):
-    pipe = cls(vqvae=None, unet=OracleUNet(), mel=ScriptedMel(), scheduler=(DDIMScheduler() if is_ddim else DDPMScheduler()))
-    pipe.set_progress_bar_config(disable=True)
-    noise = torch.randn(1, 1, 16, 16, generator=torch.Generator().manual_seed(3))   # the reference's start_step path is batch-1 only (:150)
-    kw = dict(batch_size=1, raw_audio=np.zeros(16 * 512 * 2, dtype=np.float32), slice=0, start_step=2, steps=6, noise=noise,
+def cond_call(sched):
+    """Arguments of the audio-conditioned / in-painting call (`raw_audio`, `start_step`, `mask_start_secs`,
+    `mask_end_secs`, pipeline_audio_diffusion.py:133-185) the product's pipeline is compared on."""
+    kw = dict(batch_size=1, raw_audio=np.zeros(16 * 512 * 2, dtype=np.float32), slice=0, start_step=2, steps=6,
+              noise=torch.randn(1, 1, 16, 16, generator=torch.Generator().manual_seed(3)),   # start_step is batch-1 only (:150)
               step_generator=torch.Generator().manual_seed(4), mask_start_secs=0.05, mask_end_secs=0.05, return_dict=False)
-    if is_ddim:
-        kw['eta'] = 0.5
-    images, (sr, audios) = pipe(**kw)
-    outs.append(np.stack([np.asarray(im) for im in images]))
+    if sched == "ddim":
+        kw["eta"] = 0.5
+    return kw
+
+
+@pytest.mark.parametrize("sched", ["ddpm", "ddim"])
+def test_mirrored_pipeline_equals_reference_pipeline_on_cpu(sched, monkeypatch):
+    """The product's own `AudioDiffusionPipeline.__call__` (audio_diffusion_b200/pipeline.py) against the images the
+    reference's unchanged file returned for the audio-conditioned / in-painting path (`cond_<sched>` of
+    tests/golden/reference_pipeline_cpu.npz): identical uint8 images, both driving the CPU oracle U-Net.  For DDIM also
+    the inversion (`encode`, :207-242) and `slerp` (:244-263) give the reference's numbers."""
+    Mirror = _host_u8_pipeline(monkeypatch)
+    pipe = Mirror(vqvae=None, unet=OracleUNet(), mel=ScriptedMel(), scheduler=_scheduler(sched))
+    pipe.set_progress_bar_config(disable=True)
+    images, (sr, audios) = pipe(**cond_call(sched))
+    got, gold = np.stack([np.asarray(im) for im in images]), _golden_images(f"cond_{sched}")
     assert sr == 22050 and len(audios) == 1
-assert outs[0].shape == (1, 16, 16) and np.array_equal(outs[0], outs[1]), np.abs(outs[0].astype(int) - outs[1].astype(int)).max()
-if is_ddim:   # DDIM inversion (`encode`, :207-242) and `slerp` (:244-263): same numbers from both files
-    from PIL import Image
-    rng = np.random.default_rng(9)
-    pil = [Image.fromarray(rng.integers(0, 256, (16, 16), dtype=np.uint8)) for _ in range(2)]
-    encs = []
-    for cls in (RefPipe, Mirror):
-        pipe = cls(vqvae=None, unet=OracleUNet(), mel=ScriptedMel(), scheduler=DDIMScheduler())
+    assert gold.shape == (1, 16, 16) and np.array_equal(got, gold), np.abs(got.astype(int) - gold.astype(int)).max()
+    if sched == "ddim":
+        from PIL import Image
+        rng = np.random.default_rng(9)
+        pil = [Image.fromarray(rng.integers(0, 256, (16, 16), dtype=np.uint8)) for _ in range(2)]
+        pipe = Mirror(vqvae=None, unet=OracleUNet(), mel=ScriptedMel(), scheduler=_scheduler("ddim"))
         pipe.set_progress_bar_config(disable=True)
-        encs.append(pipe.encode(pil, steps=5))
-    assert encs[0].shape == (2, 1, 16, 16) and torch.equal(encs[0], encs[1])
-    a, b = torch.randn(4, 4, generator=torch.Generator().manual_seed(1)), torch.randn(4, 4, generator=torch.Generator().manual_seed(2))
-    assert torch.equal(RefPipe.slerp(a, b, 0.3), Mirror.slerp(a, b, 0.3))
-print('ok')
-"""
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
-    assert r.returncode == 0 and "ok" in r.stdout, (r.stdout + r.stderr)[-3000:]
+        enc = pipe.encode(pil, steps=5)
+        assert enc.shape == (2, 1, 16, 16) and torch.equal(enc, torch.from_numpy(_golden_images("encode_ddim")))
+        a = torch.randn(4, 4, generator=torch.Generator().manual_seed(1))
+        b = torch.randn(4, 4, generator=torch.Generator().manual_seed(2))
+        assert torch.equal(Mirror.slerp(a, b, 0.3), torch.from_numpy(_golden_images("slerp")))
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference sources not present (GPU box)")
+MEL_CASES = [(256, 256, 512), (64, 64, 1024), (96, 32, 256)]     # (x_res, y_res, hop_length)
+
+
 def test_mel_host_logic_equals_reference_mel():
     """Slicing / padding / resolution bookkeeping of the engine's `Mel` against the reference's own `audiodiffusion/mel.py`
-    class (imported unchanged through the shim; its librosa-backed transforms are not called): mel.py:80-133."""
+    class (mel.py:80-133) on the same seeded audio: sizes, dtype and the bytes of the padded audio and of every slice,
+    as tests/golden/mel_host_logic.json records them."""
+    from audio_diffusion_b200.mel import Mel
+    with open(os.path.join(GOLDEN, "mel_host_logic.json")) as f:
+        cases = iter(json.load(f)["cases"])
+    rng = np.random.default_rng(0)
+    for (x_res, y_res, hop) in MEL_CASES:
+        for n in [10, x_res * hop - 1, x_res * hop, 3 * x_res * hop + 17]:
+            c = next(cases)
+            assert (c["x_res"], c["y_res"], c["hop_length"], c["n"]) == (x_res, y_res, hop, n)
+            b = Mel(x_res=x_res, y_res=y_res, hop_length=hop)
+            b.load_audio(raw_audio=rng.standard_normal(n).astype(np.float32))
+            assert (b.slice_size, b.n_mels, b.get_sample_rate()) == (c["slice_size"], c["n_mels"], c["sample_rate"])
+            assert b.get_number_of_slices() == c["slices"], (x_res, n)
+            assert len(b.audio) == c["audio_len"] and str(b.audio.dtype) == c["audio_dtype"]
+            assert hashlib.sha256(b.audio.tobytes()).hexdigest() == c["audio_sha256"]
+            slices = hashlib.sha256()
+            for s in range(b.get_number_of_slices()):
+                slices.update(b.get_audio_slice(s).tobytes())
+            assert slices.hexdigest() == c["slices_sha256"]
+        b.set_resolution(32, 16)
+        assert [b.x_res, b.y_res, b.n_mels, b.slice_size] == c["after_set_resolution_32_16"]
+    assert next(cases, None) is None
+
+
+def test_model_mixin_round_trip_and_conditional_unet_surface(tmp_path):
+    """SURVEY §8 f3 boundary: a model built the way the reference's audiodiffusion/audio_encoder.py builds its encoder (a
+    `diffusers` ModelMixin + ConfigMixin subclass with an argument-free constructor that holds a `diffusers.Mel`) saves and
+    loads through the shim's hub layout, and `diffusers.UNet2DConditionModel` resolves to the engine's class with exactly
+    the diffusers state-dict keys / shapes of the architecture scripts/train_unet.py:139-159 builds."""
     code = f"""
 import sys
-sys.path[:0] = [{ROOT!r}, {os.path.join(ROOT, 'audio_diffusion_b200', 'compat')!r}, {REF!r}]
-import numpy as np
-from audiodiffusion.mel import Mel as RefMel          # byte-identical reference file
-from audio_diffusion_b200.mel import Mel
-rng = np.random.default_rng(0)
-for (x_res, y_res, hop) in [(256, 256, 512), (64, 64, 1024), (96, 32, 256)]:
-    for n in [10, x_res * hop - 1, x_res * hop, 3 * x_res * hop + 17]:
-        a, b = RefMel(x_res=x_res, y_res=y_res, hop_length=hop), Mel(x_res=x_res, y_res=y_res, hop_length=hop)
-        audio = rng.standard_normal(n).astype(np.float32)
-        a.load_audio(raw_audio=audio.copy()); b.load_audio(raw_audio=audio.copy())
-        assert a.slice_size == b.slice_size and a.n_mels == b.n_mels and a.get_sample_rate() == b.get_sample_rate()
-        assert a.get_number_of_slices() == b.get_number_of_slices(), (x_res, n)
-        assert len(a.audio) == len(b.audio) and a.audio.dtype == b.audio.dtype and np.array_equal(a.audio, b.audio)
-        for s in range(a.get_number_of_slices()):
-            assert np.array_equal(a.get_audio_slice(s), b.get_audio_slice(s))
-    a.set_resolution(32, 16); b.set_resolution(32, 16)
-    assert (a.x_res, a.y_res, a.n_mels, a.slice_size) == (b.x_res, b.y_res, b.n_mels, b.slice_size)
-print('ok')
-"""
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
-    assert r.returncode == 0 and "ok" in r.stdout, (r.stdout + r.stderr)[-3000:]
-
-
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference sources not present (GPU box)")
-def test_reference_audio_encoder_and_conditional_unet_surface():
-    """SURVEY §8 f3 boundary: the reference's own audiodiffusion/audio_encoder.py runs on the shim's ModelMixin / Mel (a
-    small CNN that is not part of the denoising loop), and `diffusers.UNet2DConditionModel` resolves to the engine's class
-    with exactly the diffusers state-dict keys / shapes of the architecture scripts/train_unet.py:139-159 builds."""
-    code = f"""
-import sys, tempfile
-sys.path[:0] = [{ROOT!r}, {os.path.join(ROOT, 'audio_diffusion_b200', 'compat')!r}, {REF!r}]
+sys.path[:0] = [{ROOT!r}, {os.path.join(ROOT, 'audio_diffusion_b200', 'compat')!r}]
 import torch
-from audiodiffusion.audio_encoder import AudioEncoder          # byte-identical reference file
-enc = AudioEncoder().eval()
+from diffusers import ConfigMixin, Mel, ModelMixin
+
+class Encoder(ModelMixin, ConfigMixin):
+    def __init__(self):
+        super().__init__()
+        self.mel = Mel(x_res=216, y_res=96)
+        self.conv = torch.nn.Sequential(torch.nn.Conv2d(1, 8, 3, padding=1), torch.nn.BatchNorm2d(8), torch.nn.ReLU(),
+                                        torch.nn.MaxPool2d(4), torch.nn.Dropout(0.2))
+        self.embedding = torch.nn.Linear(8 * 24 * 54, 100)
+
+    def forward(self, x):
+        return self.embedding(self.conv(x).flatten(1))
+
+torch.manual_seed(0)
+enc = Encoder().eval()
 y = enc(torch.rand(2, 1, 96, 216))
 assert y.shape == (2, 100)
-d = tempfile.mkdtemp()
+d = {str(tmp_path / 'enc')!r}
 enc.save_pretrained(d)
-again = AudioEncoder.from_pretrained(d).eval()
+again = Encoder.from_pretrained(d).eval()
 assert torch.equal(again(torch.ones(1, 1, 96, 216)), enc(torch.ones(1, 1, 96, 216)))
 from diffusers import UNet2DConditionModel
-from audiodiffusion.pipeline_audio_diffusion import UNet2DConditionModel as seen_by_pipeline
-assert seen_by_pipeline is UNet2DConditionModel
+from audio_diffusion_b200.unet_cond import UNet2DConditionModel as engine_class
+assert engine_class is UNet2DConditionModel
 u = UNet2DConditionModel(sample_size=(32, 32), in_channels=1, out_channels=1, layers_per_block=2,
                          block_out_channels=(128, 256, 512, 512),
                          down_block_types=("CrossAttnDownBlock2D",) * 3 + ("DownBlock2D",),
@@ -396,3 +405,22 @@ def test_bench_extras_formatting():
     assert abs(out["C3_ddim50"]["value"] - 128 / (50 * 0.035 + 0.07)) < 1e-9
     assert abs(out["C5_train"]["value"] - 32 / 0.051) < 1e-9 and abs(out["C5_train"]["exposed_allreduce_ms"] - 1.0) < 1e-6
     assert out["B1_latency"]["ms_per_step"] == 4.4 and out["mel_codec"]["decode_frac"] < 1
+
+
+def test_bench_dump_outputs(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float32 .npy files; a tensor over the size cap keeps the same seeded rows on every call."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    small = torch.randn(3, 1, 4, 4, dtype=torch.float64)
+    bench.dump_outputs(str(tmp_path / "a"), {"sample": small})
+    got = np.load(tmp_path / "a" / "sample.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, small.float().numpy())
+    monkeypatch.setattr(bench, "MAX_DUMP_BYTES", 5 * 16 * 4)                 # room for 5 of the 12 samples
+    big = torch.randn(12, 1, 4, 4)
+    for d in ("b", "c"):
+        bench.dump_outputs(str(tmp_path / d), {"sample": big})
+    b, c = np.load(tmp_path / "b" / "sample.npy"), np.load(tmp_path / "c" / "sample.npy")
+    assert b.shape == (5, 1, 4, 4) and b.nbytes <= bench.MAX_DUMP_BYTES and np.array_equal(b, c)
+    assert all(any(np.array_equal(r, s) for s in big.numpy()) for r in b)

@@ -1,22 +1,25 @@
-"""The UNCHANGED reference training script (scripts/train_unet.py) driven end to end on the engine's import surfaces
-(`audio_diffusion_b200/compat`: diffusers, librosa, accelerate) through `python -m audio_diffusion_b200.compat.run`:
-two epochs on a synthetic on-disk dataset, `save_pretrained`, then a resumed run with `--from_pretrained` and
-`--start_epoch` (train_unet.py:106-111, :216-224, :302-303).
+"""A training script driven end to end on the engine's import surfaces (`audio_diffusion_b200/compat`: diffusers,
+accelerate) through `python -m audio_diffusion_b200.compat.run`: two epochs on a synthetic on-disk dataset,
+`save_pretrained`, then a resumed run with `--from_pretrained` and `--start_epoch`.
 
-This container has no GPU and the product's UNet2DModel has no CPU path, so `diffusers.UNet2DModel` is overlaid by a
-test-only autograd module backed by the oracle (tests/shims/cpu_unet); everything else — Accelerator, schedulers, EMA,
-LR schedule, pipeline save / load, Mel — is the product code the GPU run uses.  Skips where /root/reference is absent."""
+The script is tests/shims/train_unet.py, written against the same import surfaces as the upstream
+scripts/train_unet.py.  With AUDIO_DIFFUSION_SRC naming an unchanged teticio/audio-diffusion checkout, the upstream
+script runs instead, byte-identical (train_unet.py:106-111, :216-224, :302-303).
+
+The product's UNet2DModel has no CPU path, so `diffusers.UNet2DModel` is overlaid by a test-only autograd module backed
+by the oracle (tests/shims/cpu_unet); everything else — Accelerator, schedulers, EMA, LR schedule, pipeline save / load,
+Mel — is the product code the GPU run uses."""
 import json
 import os
 import subprocess
 import sys
 
 import numpy as np
-import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
-SCRIPT = os.path.join(REF, "scripts", "train_unet.py")
+REF = os.environ.get("AUDIO_DIFFUSION_SRC")
+SCRIPT = (os.path.join(REF, "scripts", "train_unet.py") if REF else
+          os.path.join(ROOT, "tests", "shims", "train_unet.py"))
 
 
 def _run(args, tmp_path, timeout=900):
@@ -28,7 +31,6 @@ def _run(args, tmp_path, timeout=900):
     return r
 
 
-@pytest.mark.skipif(not os.path.isfile(SCRIPT), reason="reference sources not present (GPU box)")
 def test_unchanged_train_script_two_epochs_then_resume(tmp_path):
     import datasets
     from PIL import Image
@@ -38,7 +40,7 @@ def test_unchanged_train_script_two_epochs_then_resume(tmp_path):
     data = tmp_path / "data"
     datasets.DatasetDict({"train": ds}).save_to_disk(str(data))
     out = tmp_path / "model"
-    common = ["--dataset_name", str(data), "--output_dir", str(out), "--train_batch_size", "2", "--eval_batch_size", "1",
+    common = ["--dataset_name", str(data), "--output_dir", str(out), "--train_batch_size", "2",
               "--lr_warmup_steps", "2", "--hop_length", "512"]
     _run(common + ["--num_epochs", "2", "--gradient_accumulation_steps", "2"], tmp_path)
     # the directory the script wrote follows the upstream layout (model_index.json with diffusers / audio_diffusion names)
